@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — CSR SpMV throughput (BASELINE.json metric) on B200, one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -49,6 +49,8 @@ import numpy as np  # noqa: E402
 METRIC = "csr_spmv_fp64_gflops"
 UNIT = "GFLOP/s"
 SEED = 1234
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE_ROWS = 1 << 22     # 32 MB of float64
 
 
 def parse():
@@ -62,7 +64,14 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the banded / cg / spgemm / powerlaw / cusparse / cpu legs")
     ap.add_argument("--spgemm-scale", type=int, default=0, help="R-MAT scale of the SpGEMM leg (0 = 18 at N=1, 20 at N>=4)")
     ap.add_argument("--pl-rows", type=int, default=8_000_000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the y of the last step to DIR/y.npy (float64; a fixed sample "
+                         f"of {DUMP_SAMPLE_ROWS} rows drawn with seed {SEED} when all of y exceeds "
+                         f"{DUMP_MAX_BYTES >> 20} MB), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 def workload_name(args):
@@ -181,6 +190,17 @@ def peaks():
         return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+def dump_outputs(out_dir, y):
+    """Write the full result vector y as out_dir/y.npy in float64, or, when it exceeds DUMP_MAX_BYTES, its
+    values at DUMP_SAMPLE_ROWS rows drawn with SEED (sorted): the same rows for every build and rank count."""
+    y = np.asarray(y, dtype=np.float64)
+    if y.nbytes > DUMP_MAX_BYTES:
+        rows = np.sort(np.random.default_rng(SEED).choice(y.size, size=DUMP_SAMPLE_ROWS, replace=False))
+        y = y[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "y.npy"), y)
+
+
 def known_traffic(tag):
     """dram bytes/launch from the committed ncu --set full capture (profiles/), or None."""
     try:
@@ -239,7 +259,9 @@ def run_reference(args):
     if rank != 0:
         return
     k, n = args.nnz_per_row, args.rows
-    info, _ = cpu_spmv_full(n, k, budget_s=max(4.0, 0.5 * args.steps), warm=max(1, min(args.warmup, 3)))
+    info, (_, _, _, _, y) = cpu_spmv_full(n, k, budget_s=max(4.0, 0.5 * args.steps), warm=max(1, min(args.warmup, 3)))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y)
     dt = info["seconds_per_spmv"]
     gflops = 2.0 * n * k / dt / 1e9
     sample = (f"the full {n}x{n} matrix ({n * k} nnz) per step, int64 column ids, identical to the GPU arm's matrix "
@@ -307,6 +329,11 @@ def run_b200(args):
     total_ms, per = timed_steps(lambda: A.dot_local(x, out=y_loc), args.steps, args.warmup, dist)
     # the counter spans warm-up + timed calls (same launches per call): keep the timed share
     launches = (_native.launch_count() - launches0) * args.steps // (args.steps + args.warmup)
+    if args.dump_outputs:
+        y_all = dist.allgather_rows(y_loc, bounds)      # collective: every rank takes part
+        if rank == 0:
+            dump_outputs(args.dump_outputs, y_all.cpu().numpy())
+        del y_all
     ms_per_step = total_ms / args.steps
     value = 2.0 * nnz_total / (ms_per_step * 1e-3) / 1e9
 
