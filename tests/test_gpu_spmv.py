@@ -162,17 +162,21 @@ def test_spmv_ragged_and_empty_rows():
 
 @pytest.mark.parametrize("tile", ["1024", "2048", "4096"])
 def test_spmv_tile_sizes_banded_and_random(monkeypatch, tile):
-    # the tile size is read once per process by the library; exercise via subprocess-free path:
-    # plans created in this process use the default, so only assert correctness for the default
+    # 1024 / 2048: pipe kernel; 4096: tile kernel (IPT 16).  The plan's window statistic is the same for
+    # every tile size: a tile of the banded matrix spans ~4096/51 rows, far inside the 1024-element window
+    monkeypatch.setenv("B2S_SPMV_TILE_NNZ", tile)
     d, c, p = gen.banded_csr_arrays(20011, 51)
     S = sp.csr_array((d, c, p), shape=(20011, 20011))
     A, x, y = _check(S)
     info = A._block().plan.info()
-    assert info["window_tiles"] == info["ntiles"]  # banded → every tile stages its x window (TMA)
+    assert info["tile_nnz"] == int(tile)
+    assert info["window_tiles"] == info["ntiles"]  # banded → every tile stages its x window
     d, c, p = gen.random_csr_fixed(30000, 40000, 50, seed=11)
     S = sp.csr_array((d, c, p), shape=(30000, 40000))
     A, x, y = _check(S)
-    assert A._block().plan.info()["window_tiles"] == 0
+    info = A._block().plan.info()
+    assert info["tile_nnz"] == int(tile)
+    assert info["window_tiles"] == 0
 
 
 def test_spmv_2d_x_and_out_rules():
