@@ -596,6 +596,8 @@ static int symbolic_typed(int64_t nrowsA, int64_t ncolsB, const int64_t* a_ptr, 
   SpgemmWs W = carve_ws(workspace, nrowsA);
   B2S_CUDA_TRY(cudaMemsetAsync(W.counters, 0, 16 * 8, st));
   if (nrowsA == 0) {
+    // an empty row block still has c_indptr[0] = nnz(C) = 0 (the caller may have allocated it uninitialised)
+    B2S_CUDA_TRY(cudaMemsetAsync(c_ptr, 0, sizeof(int64_t), st));
     if (out_nnzC) *out_nnzC = 0;
     if (out_products) *out_products = 0;
     return B2S_OK;
